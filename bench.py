@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- mocap frame-sets/s of the B200 marker-tracking core (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (S1 blob detection -> S2 epipolar matching -> S3 DLT
 triangulation + reprojection error, one launch group per batch) over one batch of synthetic
@@ -338,6 +338,34 @@ def committed_traffic(workload, kernel_prefix):
     return int(t["dram_bytes_read"]) + int(t["dram_bytes_write"]), f"profiles/traffic_{workload}.json <- {t.get('source')}"
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, out, ba_R=None, ba_t=None):
+    """What the caller of the timed path receives for the last timed step, one <name>.npy per array: the track
+    buffers of mocap_pipeline_dev (obj, err, n, flags, and track_xy when S4 runs) and the refined poses of that
+    step's bundle adjustments.  Slots at and past n[b] hold no result and are written as zero, so that two builds
+    can be compared array for array."""
+    n = out["n"].cpu().numpy()
+    unused = np.arange(out["obj"].shape[1])[None, :] >= n[:, None]                 # [B, R]
+    arrays = {"obj": out["obj"].cpu().numpy().astype(np.float64), "err": out["err"].cpu().numpy().astype(np.float64),
+              "n": n.astype(np.float32), "flags": out["flags"].cpu().numpy().astype(np.float32)}
+    arrays["obj"][unused] = 0
+    arrays["err"][unused] = 0
+    if "track_xy" in out:
+        arrays["track_xy"] = out["track_xy"].cpu().numpy().astype(np.float32)
+        arrays["track_xy"][unused] = 0
+    if ba_R is not None:
+        arrays["ba_R"] = np.stack([r.cpu().numpy() for r in ba_R]).astype(np.float64)
+        arrays["ba_t"] = np.stack([t.cpu().numpy() for t in ba_t]).astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -530,6 +558,9 @@ def run_gpu_arm(args):
 
     # ---- checks on every rank: no capacity overflow anywhere in the timed batch; the first frame-sets against the oracle
     out = outs[(step_no[0] - 1) % n_bufs]
+    if args.dump_outputs and rank == 0:                  # before the e2e leg, which reuses the S4 buffers
+        last = ((step_no[0] - 1) % n_bufs) * n_sub if with_ba else 0
+        dump_outputs(args.dump_outputs, out, *((ba_R[last:last + n_sub], ba_t[last:last + n_sub]) if with_ba else ()))
     flags_set = int((out["flags"] != 0).sum().item())
     problems = []
     if flags_set:
@@ -711,7 +742,13 @@ def main():
     ap.add_argument("--no-ba", action="store_true", help="c8m16 at N = 1 without S4 (the S1-S3 figure of the config-3 shape)")
     ap.add_argument("--profile", action="store_true",
                     help="resident steps only (no e2e, no CPU baseline): for runs under ncu; prints no bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy, float32 / float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 implementation")
     if args.workload == "c8m16":
         global N_CAM, N_MARKERS, BATCH, POOL, MAX_ROOTS, MAX_GROUPS, WITH_BA
         N_CAM, N_MARKERS, BATCH, POOL, MAX_ROOTS, MAX_GROUPS, WITH_BA = 8, 16, 4000, 4000, 64, 1 << 16, True

@@ -1,6 +1,7 @@
 """Loader for the UNMODIFIED reference implementation (test infrastructure only).
 
-This module imports ``/root/reference/computer_code/api/helpers.py`` as it lies,
+This module imports ``computer_code/api/helpers.py`` of a jyjblrd/Low-Cost-Mocap
+checkout named by the ``LOW_COST_MOCAP_DIR`` environment variable, as it lies,
 with the three shims SURVEY.md §8(c) lists:
 
 * a one-class ``pseyepy`` stub (the module is imported at helpers.py:12 and a
@@ -10,17 +11,16 @@ with the three shims SURVEY.md §8(c) lists:
 * ``cv2.sfm`` provided by :mod:`oracle.sfm_shim` (opencv_contrib is not
   installed; that boundary is parity-UNPINNED, see DESIGN.md).
 
-``/root/reference`` exists only in the build container, never on the GPU box,
-so nothing here may be imported by ``-m gpu`` tests, ``smoke()`` or ``bench.py``.
-It is used by ``tests/golden/make_golden.py`` (to write the committed golden
-vectors) and by the CPU-only tests that pin ``oracle/ref_port.py`` against the
-real reference whenever the reference tree is present.
+The reference is not part of this repository, so nothing here may be imported
+by the tests, ``smoke()`` or ``bench.py``.  It is used only by
+``tests/golden/make_golden.py``, which writes the committed golden vectors that
+the tests compare against.
 """
 import os
 import sys
 import types
 
-REFERENCE_API_DIR = "/root/reference/computer_code/api"
+REFERENCE_API_DIR = os.path.join(os.environ.get("LOW_COST_MOCAP_DIR", ""), "computer_code", "api")
 
 
 def reference_available() -> bool:
@@ -43,7 +43,7 @@ def load_reference(num_cameras: int, intrinsic_matrix=None):
     from . import sfm_shim
 
     if not reference_available():
-        raise RuntimeError("reference tree not present (expected only in the build container)")
+        raise RuntimeError("reference tree not found: set LOW_COST_MOCAP_DIR to a jyjblrd/Low-Cost-Mocap checkout")
 
     if _cached is None:
         stub = types.ModuleType("pseyepy")

@@ -5,16 +5,15 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and the ``cpu_baseline`` /
 checker or as the timed CPU baseline, never as a product path.
 
 The reference is plain Python on top of cv2 / numpy / scipy
-(/root/reference/computer_code/api/helpers.py).  It cannot travel to the GPU box,
-so this file restates, stage by stage, what it computes, calling the SAME
+(computer_code/api/helpers.py of jyjblrd/Low-Cost-Mocap).  It is not part of this
+repository, so this file restates, stage by stage, what it computes, calling the SAME
 third-party routines at the same precision (cv2.findContours/moments,
 cv2.computeCorrespondEpilines, cv2.projectPoints, scipy.linalg.svd,
 scipy.optimize.least_squares) so both the numbers and the CPU cost are those of
 the reference.  Pinning: ``tests/test_oracle_pinned.py`` checks every function
-here against (a) the real reference imported via ``oracle/ref_harness.py`` when
-``/root/reference`` is present and (b) the committed vectors in
-``tests/golden/*.npz`` that ``tests/golden/make_golden.py`` wrote by running
-the real reference.  The three ``cv2.sfm`` calls are restated in
+here against the committed vectors in ``tests/golden/*.npz`` that
+``tests/golden/make_golden.py`` wrote by running the real reference (imported via
+``oracle/ref_harness.py``).  The three ``cv2.sfm`` calls are restated in
 ``oracle/sfm_shim.py`` -- that boundary alone is parity-UNPINNED.
 
 Stage map (reference file:line):

@@ -1,8 +1,8 @@
 """Writes tests/golden/*.npz by running the REAL reference
-(/root/reference/computer_code/api/helpers.py, imported unmodified through
-oracle/ref_harness.py) on seeded synthetic inputs.  Run in the build container:
+(computer_code/api/helpers.py of a jyjblrd/Low-Cost-Mocap checkout, imported
+unmodified through oracle/ref_harness.py) on seeded synthetic inputs:
 
-    python tests/golden/make_golden.py
+    LOW_COST_MOCAP_DIR=<checkout> python tests/golden/make_golden.py
 
 The vectors pin oracle/ref_port.py (tests/test_oracle_pinned.py) and the CUDA
 path (tests/test_parity_gpu.py) on the GPU box, where the reference is absent.
@@ -212,8 +212,87 @@ def ba_case(name, C, F, seed):
     print(name, "cost", cost(r0), "->", cost(rf))
 
 
+def reference_calls_case(name):
+    """What the reference returns for the inputs of the port-versus-reference tests in tests/test_oracle_pinned.py:
+    S1-S3 on three frame-sets, one S4 residual vector, locate_objects, make_square, the camera chain that index.py's
+    calculate_camera_pose hands to bundle_adjustment, and which hot-path names its two modules hold."""
+    import hashlib
+    import cv2
+    from oracle.ref_harness import load_reference_index
+    api = importlib.import_module("low-cost-mocap_b200.api")
+    z = {}
+    # S1-S3: 4 cameras, 6 markers, 3 frame-sets of the synthetic stream (seed 42)
+    C, M, B = 4, 6, 3
+    helpers, cams = load_reference(C)
+    frames, _, poses, _ = synth.make_frame_pool(C, M, B, seed=42)
+    blob_xy = np.full((B, C, MAXB, 2), -1, dtype=np.int32)
+    blob_n = np.zeros((B, C), dtype=np.int32)             # 0: _find_dot returned [[None, None]]
+    obj = np.full((B, MAXR, 3), np.nan)
+    err = np.full((B, MAXR), np.nan)
+    nroot = np.zeros((B,), dtype=np.int32)
+    for b in range(B):
+        pts = [cams._find_dot(np.repeat(frames[b, c][:, :, None], 3, axis=2).copy())[1] for c in range(C)]
+        for c, p in enumerate(pts):
+            real = [q for q in p if q[0] is not None]
+            assert len(real) == len(p) or p == [[None, None]]
+            blob_n[b, c] = len(real)
+            for i, q in enumerate(real):
+                blob_xy[b, c, i] = q
+        e, o, _ = helpers.find_point_correspondance_and_object_points([list(map(list, p)) for p in pts], poses, [None] * C)
+        nroot[b] = len(e)
+        obj[b, :len(e)] = np.asarray(o, dtype=np.float64).reshape(-1, 3)
+        err[b, :len(e)] = e
+    z.update(pipe_blob_xy=blob_xy, pipe_blob_n=blob_n, pipe_obj=obj, pipe_err=err, pipe_nroot=nroot)
+    # S4 residual vector: 3 cameras, 12 points (seed 2), start perturbed with seed 3
+    helpers, cams = load_reference(3)
+    obs, poses, K, _ = synth.make_tracks(3, 12, seed=2)
+    start = synth.perturb_poses(poses, seed=3)
+    X = helpers.triangulate_points(obs, start)
+    z["ba_r"] = helpers.calculate_reprojection_errors(obs, X, start).astype(np.float32)
+    # locate_objects on 30 seeded drone layouts
+    helpers, _ = load_reference(2)
+    counts, pos, heading, error, drone = [], [], [], [], []
+    for seed in range(30):
+        pts, errs = synth.make_drone_points(1 + seed % 3, seed % 5, seed=seed)
+        found = helpers.locate_objects(pts.copy(), errs.copy())
+        counts.append(len(found))
+        for f in found:
+            pos.append(f["pos"]); heading.append(f["heading"]); error.append(f["error"]); drone.append(f["droneIndex"])
+    z.update(loc_counts=np.array(counts, dtype=np.int32), loc_pos=np.array(pos, dtype=np.float64).reshape(-1, 3),
+             loc_heading=np.array(heading, dtype=np.float64), loc_error=np.array(error, dtype=np.float64),
+             loc_drone=np.array(drone, dtype=np.int32))
+    # make_square of a 240x320 noise frame (seed 0): the output is incompressible noise, so its digest is stored
+    helpers, _ = load_reference(1)
+    sq = helpers.make_square(np.random.default_rng(0).integers(0, 256, size=(240, 320, 3), dtype=np.uint8))
+    z.update(square_shape=np.array(sq.shape), square_sha256=np.array(hashlib.sha256(np.ascontiguousarray(sq).tobytes()).hexdigest()))
+    # index.py calculate_camera_pose: 3 cameras, 40 frames (seed 8), cv2 RNG seed 0; bundle_adjustment intercepted
+    index, helpers, cams = load_reference_index(3)
+    obs, poses, K, _ = synth.make_tracks(3, 40, seed=8, missing_frac=0.15)
+    captured = {}
+
+    def fake_ba(image_points, camera_poses, sio):
+        captured["poses"] = camera_poses
+        return camera_poses
+    real_ba, real_ser = index.bundle_adjustment, index.camera_pose_to_serializable
+    index.bundle_adjustment = fake_ba
+    index.camera_pose_to_serializable = lambda p: p
+    try:
+        cv2.setRNGSeed(0)
+        index.calculate_camera_pose({"cameraPoints": obs.tolist()})
+    finally:
+        index.bundle_adjustment, index.camera_pose_to_serializable = real_ba, real_ser
+    z.update(calib_R=np.stack([np.array(p["R"], dtype=np.float64) for p in captured["poses"]]),
+             calib_t=np.stack([np.array(p["t"], dtype=np.float64).reshape(3) for p in captured["poses"]]))
+    z.update(helpers_names=np.array([n for n in api.PATCHED_NAMES if hasattr(helpers, n)]),
+             index_names=np.array([n for n in api.PATCHED_NAMES if hasattr(index, n)]))
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **z)
+    print(name, "roots", nroot.tolist(), "objects", int(sum(counts)), "index holds", z["index_names"].tolist())
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["pipe", "blobs", "rings", "tri", "ba"]
+    which = sys.argv[1:] or ["pipe", "blobs", "rings", "tri", "ba", "calls"]
+    if "calls" in which:
+        reference_calls_case("reference_calls")
     if "pipe8" in which:
         pipeline_case("pipe_c8_m16", 8, 16, 100, seed=0)
     if "pipe" in which:

@@ -10,7 +10,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from tests.util import ROOT, load_golden
+from tests.util import ROOT, compile_shared, load_golden
 
 PIPE_CASES = ["pipe_c2_m1", "pipe_c4_m4", "pipe_c8_m16"]
 
@@ -24,7 +24,7 @@ CUDA_INC = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "include
 def blob_emu():
     src = os.path.join(HC, "blob_emu_host.cpp")
     out = os.path.join(HC, "libblob_emu.so")
-    subprocess.check_call(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
+    compile_shared(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
                            "-fno-strict-aliasing", "-o", out, src])
     lib = ctypes.CDLL(out)
 
@@ -141,7 +141,7 @@ ERR_RTOL = 1e-9
 def match_emu():
     src = os.path.join(HC, "match_emu_host.cpp")
     out = os.path.join(HC, "libmatch_emu.so")
-    subprocess.check_call(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
+    compile_shared(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
                            "-fno-strict-aliasing", "-o", out, src])
     lib = ctypes.CDLL(out)
 
@@ -270,7 +270,7 @@ def test_matcher_device_code_capacity_flags(match_emu):
 def fused_emu():
     src = os.path.join(HC, "fused_emu_host.cpp")
     out = os.path.join(HC, "libfused_emu.so")
-    subprocess.check_call(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
+    compile_shared(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
                            "-fno-strict-aliasing", "-o", out, src])
     lib = ctypes.CDLL(out)
 
@@ -532,10 +532,10 @@ def test_phased_kernel_on_host_equals_single_pass_kernel(fused_emu):
 @pytest.fixture(scope="module")
 def ba_emu():
     out = os.path.join(HC, "libba_dev_emu.so")
-    subprocess.check_call(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
+    compile_shared(["g++", "-std=c++20", "-O2", "-shared", "-fPIC", "-pthread", "-I" + CUDA_INC, "-Wno-attributes",
                            "-fno-strict-aliasing", "-o", out, os.path.join(HC, "ba_dev_emu_host.cpp")])
     model = os.path.join(HC, "libba_host.so")
-    subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-o", model, os.path.join(HC, "ba_host.cpp"), "-lm"])
+    compile_shared(["g++", "-O2", "-shared", "-fPIC", "-o", model, os.path.join(HC, "ba_host.cpp"), "-lm"])
     emu, host = ctypes.CDLL(out), ctypes.CDLL(model)
     emu.hc_ba_solve_dev.argtypes = [ctypes.c_void_p] * 2 + [ctypes.c_int] * 2 + [ctypes.c_void_p] * 3 + [ctypes.c_double] + [ctypes.c_int] * 6 + [ctypes.c_void_p]
     host.hc_bundle_adjust.argtypes = [ctypes.c_void_p] * 2 + [ctypes.c_int] * 2 + [ctypes.c_void_p] * 3 + [ctypes.c_double, ctypes.c_int, ctypes.c_void_p, ctypes.c_int]

@@ -11,7 +11,7 @@ import sys
 import numpy as np
 import pytest
 
-from tests.util import ROOT, load_golden
+from tests.util import ROOT, compile_shared, load_golden
 
 pkg = importlib.import_module("low-cost-mocap_b200")
 _lib = importlib.import_module("low-cost-mocap_b200._lib")
@@ -125,7 +125,7 @@ def geom_host():
     out = os.path.join(ROOT, "tests", "hostcheck", "libgeom_host.so")
     if not os.path.exists(out) or os.path.getmtime(out) < max(os.path.getmtime(src), os.path.getmtime(
             os.path.join(ROOT, "low-cost-mocap_b200", "csrc", "geom.cuh"))):
-        subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-ffp-contract=off", "-o", out, src, "-lm"])
+        compile_shared(["g++", "-O2", "-shared", "-fPIC", "-ffp-contract=off", "-o", out, src, "-lm"])
     return ctypes.CDLL(out)
 
 
@@ -166,7 +166,7 @@ def test_header_is_plain_c_and_example_links(built_lib, tmp_path):
 def ba_host():
     src = os.path.join(ROOT, "tests", "hostcheck", "ba_host.cpp")
     out = os.path.join(ROOT, "tests", "hostcheck", "libba_host.so")
-    subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-ffp-contract=off", "-o", out, src, "-lm"])
+    compile_shared(["g++", "-O2", "-shared", "-fPIC", "-ffp-contract=off", "-o", out, src, "-lm"])
     return ctypes.CDLL(out)
 
 
@@ -211,7 +211,7 @@ def test_ba_host_model_reaches_reference_quality(ba_host):
 def preproc_host():
     src = os.path.join(ROOT, "tests", "hostcheck", "preproc_host.cpp")
     out = os.path.join(ROOT, "tests", "hostcheck", "libpreproc_host.so")
-    subprocess.check_call(["g++", "-O2", "-shared", "-fPIC", "-fno-strict-aliasing", "-o", out, src])
+    compile_shared(["g++", "-O2", "-shared", "-fPIC", "-fno-strict-aliasing", "-o", out, src])
     return ctypes.CDLL(out)
 
 

@@ -1,11 +1,10 @@
-"""Pins oracle/ref_port.py: (a) against the committed golden vectors written by the
-real reference (tests/golden/make_golden.py), (b) against the live reference when
-/root/reference is present (build container only).  CPU only."""
+"""Pins oracle/ref_port.py against the committed golden vectors that tests/golden/make_golden.py wrote by running
+the real reference: its pipeline outputs (pipe_*, tri_*, ba_*) and, in reference_calls.npz, what its functions
+returned for the inputs of the *_live_reference tests below.  CPU only."""
 import numpy as np
 import pytest
 
 from oracle.ref_port import RefPort
-from oracle import ref_harness
 from tests.util import load_golden, poses_from, obs_from, as3
 
 PIPE_CASES = ["pipe_c2_m1", "pipe_c4_m4", "pipe_c8_m16"]
@@ -69,31 +68,33 @@ def test_triangulate_needs_two_views():
     assert port.find_dot(np.zeros((480, 640, 3), np.uint8)) == [[None, None]]
 
 
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
+def _reference_calls():
+    return load_golden("reference_calls")
+
+
 def test_port_equals_live_reference(synth):
+    """S1-S3 of the port against what the reference returned for the same three frame-sets."""
+    z = _reference_calls()
     C, M = 4, 6
-    helpers, cams = ref_harness.load_reference(C)
     frames, truth, poses, K = synth.make_frame_pool(C, M, 3, seed=42)
     port = RefPort([K] * C)
     for b in range(3):
-        ref_pts = [cams._find_dot(as3(frames[b, c]))[1] for c in range(C)]
+        ref_pts = [[list(map(int, p)) for p in z["pipe_blob_xy"][b, c, :z["pipe_blob_n"][b, c]]] or [[None, None]] for c in range(C)]
         my_pts = [port.find_dot(as3(frames[b, c])) for c in range(C)]
         assert ref_pts == my_pts
-        e, o, _ = helpers.find_point_correspondance_and_object_points([list(map(list, p)) for p in ref_pts], poses, [None] * C)
         e2, o2, _ = port.match_and_triangulate(my_pts, poses)
-        assert np.array_equal(e, e2)
-        assert np.array_equal(np.asarray(o, dtype=np.float64), np.asarray(o2, dtype=np.float64))
+        k = int(z["pipe_nroot"][b])
+        assert np.array_equal(z["pipe_err"][b, :k], e2)
+        assert np.array_equal(z["pipe_obj"][b, :k], np.asarray(o2, dtype=np.float64).reshape(-1, 3))
 
 
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
 def test_ba_residuals_equal_live_reference(synth):
     C = 3
-    helpers, cams = ref_harness.load_reference(C)
+    z = _reference_calls()
     obs, poses, K, _ = synth.make_tracks(C, 12, seed=2)
     start = synth.perturb_poses(poses, seed=3)
     port = RefPort([K] * C)
-    X = helpers.triangulate_points(obs, start)
-    r_ref = helpers.calculate_reprojection_errors(obs, X, start).astype(np.float32)
+    r_ref = z["ba_r"]
     x0 = port.poses_to_params(start)
     r = port.ba_residuals(x0, obs)
     # poses -> rotvec -> matrix round trip in the port: equal to float32 resolution
@@ -101,136 +102,112 @@ def test_ba_residuals_equal_live_reference(synth):
     assert np.allclose(r, r_ref, rtol=1e-5, atol=1e-6)
 
 
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
 def test_locate_objects_equals_live_reference(synth):
-    helpers, _ = ref_harness.load_reference(2)
+    z = _reference_calls()
     total = 0
     for seed in range(30):
         pts, errs = synth.make_drone_points(1 + seed % 3, seed % 5, seed=seed)
-        ref = helpers.locate_objects(pts.copy(), errs.copy())
         mine = RefPort.locate_objects(pts.copy(), errs.copy())
-        assert len(ref) == len(mine)
-        total += len(ref)
-        for a, b in zip(ref, mine):
-            assert np.array_equal(a["pos"], b["pos"]) and a["heading"] == b["heading"]
-            assert a["error"] == b["error"] and a["droneIndex"] == b["droneIndex"]
+        assert len(mine) == z["loc_counts"][seed]
+        for i, b in enumerate(mine, start=total):
+            assert np.array_equal(z["loc_pos"][i], b["pos"]) and z["loc_heading"][i] == b["heading"]
+            assert z["loc_error"][i] == b["error"] and z["loc_drone"][i] == b["droneIndex"]
+        total += len(mine)
     assert total >= 30
 
 
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
 def test_preprocess_equals_live_reference():
-    """RefPort.preprocess restates helpers.py:70-82; the live reference only exposes that chain inside
-    _camera_read (which needs camera hardware), so its pieces are compared: make_square directly, the
-    cv2 calls by construction (same functions, same arguments)."""
-    helpers, cams = ref_harness.load_reference(1)
+    """RefPort.preprocess restates helpers.py:70-82; the reference only exposes that chain inside _camera_read
+    (which needs camera hardware), so its pieces are compared: make_square against the digest of the reference's
+    output, the cv2 calls by construction (same functions, same arguments)."""
+    import hashlib
+    z = _reference_calls()
     rng = np.random.default_rng(0)
     frame = rng.integers(0, 256, size=(240, 320, 3), dtype=np.uint8)
-    assert np.array_equal(helpers.make_square(frame), RefPort.make_square(frame))
+    sq = RefPort.make_square(frame)
+    assert sq.dtype == np.uint8 and sq.shape == tuple(z["square_shape"])
+    assert hashlib.sha256(np.ascontiguousarray(sq).tobytes()).hexdigest() == str(z["square_sha256"])
 
 
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
 def test_calibrate_init_equals_live_reference(synth):
-    """index.py:229-270 through the real handler: bundle_adjustment is intercepted so that the chain it
-    is handed can be compared with the port's (same cv2 RNG seed on both sides)."""
-    import cv2
+    """index.py:229-270: the camera chain the reference's calculate_camera_pose hands to bundle_adjustment (cv2 RNG
+    seed 0) against the port's (same seed)."""
     C = 3
-    index, helpers, cams = ref_harness.load_reference_index(C)
+    z = _reference_calls()
     obs, poses, K, _ = synth.make_tracks(C, 40, seed=8, missing_frac=0.15)
-    captured = {}
-
-    def fake_ba(image_points, camera_poses, sio):
-        captured["poses"] = [{"R": np.array(p["R"], dtype=np.float64), "t": np.array(p["t"], dtype=np.float64)} for p in camera_poses]
-        return camera_poses
-    real_ba, real_ser = index.bundle_adjustment, index.camera_pose_to_serializable
-    index.bundle_adjustment = fake_ba
-    index.camera_pose_to_serializable = lambda p: p
-    try:
-        cv2.setRNGSeed(0)
-        index.calculate_camera_pose({"cameraPoints": obs.tolist()})
-    finally:
-        index.bundle_adjustment, index.camera_pose_to_serializable = real_ba, real_ser
     mine = RefPort([K] * C).calibrate_init(obs.tolist(), rng_seed=0)
-    assert len(mine) == len(captured["poses"]) == C
-    for a, b in zip(mine, captured["poses"]):
-        assert np.array_equal(np.asarray(a["R"], dtype=np.float64), b["R"])
-        assert np.array_equal(np.asarray(a["t"], dtype=np.float64).ravel(), b["t"].ravel())
+    assert len(mine) == len(z["calib_R"]) == C
+    for c, a in enumerate(mine):
+        assert np.array_equal(np.asarray(a["R"], dtype=np.float64), z["calib_R"][c])
+        assert np.array_equal(np.asarray(a["t"], dtype=np.float64).ravel(), z["calib_t"][c])
 
 
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
-def test_install_into_rebinds_the_live_reference_module():
+def _reference_shaped_modules(z):
+    """Stand-ins with the layout install_into relies on: ``helpers`` holds the hot-path names the reference's helpers
+    module holds and a ``Cameras`` singleton wrapper whose instance has ``camera_params``; ``index`` holds the names
+    the reference's index.py imported from helpers by value."""
+    import types
+
+    class Cameras:
+        def __init__(self):
+            K = [[600.0, 0.0, 320.0], [0.0, 600.0, 240.0], [0.0, 0.0, 1.0]]
+            self.camera_params = [{"intrinsic_matrix": np.array(K), "distortion_coef": np.zeros(5), "rotation": 0}
+                                  for _ in range(4)]
+
+        def _find_dot(self, img):
+            return img, [[None, None]]
+
+    class Singleton:                                   # instance() creates the decorated class once
+        def __init__(self, decorated):
+            self._decorated = decorated
+
+        def instance(self):
+            if not hasattr(self, "_instance"):
+                self._instance = self._decorated()
+            return self._instance
+
+    def cpu_function(name):
+        def f(*a):
+            raise AssertionError(f"the CPU {name} was called")
+        return f
+
+    helpers = types.ModuleType("helpers")
+    helpers.Cameras = Singleton(Cameras)
+    for n in z["helpers_names"]:
+        setattr(helpers, str(n), cpu_function(str(n)))
+    index = types.ModuleType("index")
+    for n in z["index_names"]:
+        setattr(index, str(n), getattr(helpers, str(n)))
+    return helpers, index
+
+
+def test_install_into_rebinds_reference_shaped_modules():
     """INTEGRATION.md: install_into() must replace exactly the names the reference's callers resolve at call
-    time -- the method on the class behind the Singleton wrapper and the module-level functions."""
-    import importlib
-    pkg = importlib.import_module("low-cost-mocap_b200")
-    helpers, cams = ref_harness.load_reference(4)
-    names = ["triangulate_point", "triangulate_points", "calculate_reprojection_error", "calculate_reprojection_errors",
-             "find_point_correspondance_and_object_points", "bundle_adjustment", "locate_objects"]
-    saved = {n: getattr(helpers, n) for n in names}
-    saved_fd = type(cams)._find_dot
-    try:
-        s = pkg.install_into(helpers)
-        assert len(s.intrinsics) == 4 and np.array_equal(s.intrinsics[0], np.asarray(cams.camera_params[0]["intrinsic_matrix"]))
-        assert type(cams)._find_dot is not saved_fd
-        assert cams._find_dot.__func__ is type(cams)._find_dot          # what _camera_read will call (helpers.py:87)
-        for n in names:
-            assert getattr(helpers, n) is not saved[n]
-        # without a GPU the replacements fail loudly instead of falling back
-        import torch
-        if not torch.cuda.is_available():
-            with pytest.raises(Exception):
-                helpers.triangulate_points([[[1, 2], [3, 4], [None, None], [None, None]]], [{"R": np.eye(3), "t": np.zeros(3)}] * 4)
-    finally:
-        for n in names:
-            setattr(helpers, n, saved[n])
-        type(cams)._find_dot = saved_fd
-
-
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree only exists in the build container")
-def test_install_into_reaches_the_names_index_imported_by_value(monkeypatch, synth):
-    """index.py binds bundle_adjustment / triangulate_points / calculate_reprojection_errors BY VALUE
-    (``from helpers import ...``, index.py:1), so patching ``helpers`` alone leaves the calculate-camera-pose
-    handler (index.py:254,272,274,275 -- BASELINE config 5's caller) on the CPU functions.
-    ``install_into(helpers, index)`` must re-bind them there too: the unmodified handler is run and every one of
-    the three calls has to arrive in the replacement layer (which, in this GPU-less tier, is pointed back at the
-    reference's own functions so that the handler runs to its end)."""
+    time -- the method on the class behind the Singleton wrapper, the module-level functions of helpers.py, and
+    the names index.py imported from it by value (index.py:1)."""
     import importlib
     pkg = importlib.import_module("low-cost-mocap_b200")
     api = importlib.import_module("low-cost-mocap_b200.api")
-    index, helpers, cams = ref_harness.load_reference_index(4)
-    names = list(api.PATCHED_NAMES)
-    saved_h = {n: getattr(helpers, n) for n in names}
-    saved_i = {n: getattr(index, n) for n in names if hasattr(index, n)}
-    assert set(saved_i) == {"bundle_adjustment", "triangulate_points", "calculate_reprojection_errors"}
+    z = _reference_calls()
+    assert sorted(map(str, z["helpers_names"])) == sorted(api.PATCHED_NAMES)
+    assert set(map(str, z["index_names"])) == {"bundle_adjustment", "triangulate_points", "calculate_reprojection_errors"}
+    helpers, index = _reference_shaped_modules(z)
+    cams = helpers.Cameras.instance()
+    saved = {n: getattr(helpers, n) for n in api.PATCHED_NAMES}
     saved_fd = type(cams)._find_dot
-    reached = []
-
-    def spy(name):
-        def f(*a):
-            reached.append(name)
-            return saved_h[name](*a[:-1])              # drop the session argument, run the reference's own code
-        return f
-
-    for n in names:                                    # every replacement, so that nested calls stay on the CPU here
-        monkeypatch.setattr(api, n, spy(n))
-    try:
-        pkg.install_into(helpers, index)
-        for n in saved_i:
-            assert getattr(index, n) is getattr(helpers, n) and getattr(index, n) is not saved_i[n]
-            assert getattr(index, n).__mocap_b200__
-        obs, poses, K, pts = synth.make_tracks(4, 30, seed=2, missing_frac=0.0)
-        import cv2
-        cv2.setRNGSeed(1)
-        index.socketio.events.clear()
-        index.calculate_camera_pose({"cameraPoints": obs.tolist()})
-        assert "bundle_adjustment" in reached and "calculate_reprojection_errors" in reached
-        assert reached.count("triangulate_points") >= 3 * 4 + 1       # 4 cheirality candidates per pair + the final call
-        assert index.socketio.events and index.socketio.events[-1][0][0] == "camera-pose"
-    finally:
-        for n, f in saved_h.items():
-            setattr(helpers, n, f)
-        for n, f in saved_i.items():
-            setattr(index, n, f)
-        type(cams)._find_dot = saved_fd
+    s = pkg.install_into(helpers, index)
+    assert len(s.intrinsics) == 4 and np.array_equal(s.intrinsics[0], np.asarray(cams.camera_params[0]["intrinsic_matrix"]))
+    assert type(cams)._find_dot is not saved_fd
+    assert cams._find_dot.__func__ is type(cams)._find_dot          # what _camera_read will call (helpers.py:87)
+    for n in api.PATCHED_NAMES:
+        assert getattr(helpers, n) is not saved[n] and getattr(helpers, n).__mocap_b200__
+    for n in map(str, z["index_names"]):
+        assert getattr(index, n) is getattr(helpers, n)
+    # without a GPU the replacements fail loudly instead of falling back
+    import torch
+    if not torch.cuda.is_available():
+        with pytest.raises(pkg.MocapError):
+            helpers.triangulate_points([[[1, 2], [3, 4], [None, None], [None, None]]], [{"R": np.eye(3), "t": np.zeros(3)}] * 4)
 
 
 @pytest.mark.parametrize("name", ["ba_c8", "ba_c16"])

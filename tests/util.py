@@ -1,6 +1,7 @@
 """Helpers shared by the CPU and GPU test files."""
 import importlib
 import os
+import subprocess
 
 import numpy as np
 
@@ -49,3 +50,13 @@ def obs_from(z):
 
 def as3(img):
     return np.repeat(img[:, :, None], 3, axis=2).copy()
+
+
+def compile_shared(cmd):
+    """Run a compiler command ``cmd`` (which names its output with "-o", path) so that the library appears at that
+    path only once it is complete: test processes running side by side (pytest -n) never load a half-written one."""
+    out = cmd[cmd.index("-o") + 1]
+    tmp = f"{out[:-len('.so')]}.{os.getpid()}.tmp.so"
+    subprocess.check_call([tmp if a == out else a for a in cmd])
+    os.replace(tmp, out)
+    return out
